@@ -13,6 +13,12 @@ composites its own output stream (weak scaling, no data-path collective: outputs
 `roofline`  dominant kernel: algorithmic bytes per launch / its device time (events inside the library).
 `cpu_baseline` / `--impl reference`: the CPU oracle (restatement of the reference's wgpu path; the
             reference itself is Rust + wgpu and cannot run here) timed on the host cores, bounded sample.
+
+--dump-outputs DIR  after the timed steps, writes the output planes of the last timed step as DIR/<name>.npy
+            (float32 copies of the NV12 bytes, e.g. output_1_y.npy (H, W) and output_1_uv.npy (H/2, W/2, 2)).  Inputs
+            are seeded, so the same arguments give the same inputs on every run and two builds can be compared file by
+            file.  At most 64 MB are written: a larger output keeps a fixed, seeded subset of its rows (the row numbers
+            go to <name>_rows.npy).
 """
 import argparse
 import ctypes as C
@@ -247,7 +253,7 @@ def run_reference(args, wl):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    times, desc, cores = cpu_steps(wl, max(args.steps, 5), max(args.warmup, 1))
+    times, desc, cores = cpu_steps(wl, args.steps, args.warmup)
     per_frame = float(np.median(times))
     fps = 1.0 / per_frame
     line = {"impl": "reference", "metric": metric_name(wl), "value": fps, "unit": "frames/s",
@@ -260,6 +266,24 @@ def run_reference(args, wl):
             "e2e": {"value": fps, "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
     print(json.dumps(line))
+
+
+DUMP_BYTES = 64 * 10**6   # the whole --dump-outputs set, .npy headers included
+
+
+def dump_outputs(directory, planes, budget=DUMP_BYTES):
+    """planes: {name: uint8 numpy array (rows first)}.  Writes each as float32 <name>.npy; when the set would exceed the
+    budget, every plane keeps the same seeded share of its rows and the chosen row numbers are written beside it."""
+    os.makedirs(directory, exist_ok=True)
+    header = 256   # per file, generous for an .npy header
+    total = sum(p.size * 4 + header for p in planes.values())
+    share = 1.0 if total <= budget else (budget - 2 * header * len(planes)) / (total + 8 * sum(len(p) for p in planes.values()))
+    for i, (name, p) in enumerate(planes.items()):
+        if share < 1.0:
+            rows = np.sort(np.random.default_rng(1000 + i).choice(len(p), max(1, int(len(p) * share)), replace=False))
+            np.save(os.path.join(directory, f"{name}_rows.npy"), rows.astype(np.float64))
+            p = p[rows]
+        np.save(os.path.join(directory, f"{name}.npy"), p.astype(np.float32))
 
 
 class _DevMem:
@@ -431,7 +455,13 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="N > 1: skip the cfg4 (NVLink exchange) leg")
     ap.add_argument("--exchange", default="all", choices=["all", "nccl", "peer_copy", "peer_direct"],
                     help="N > 1, cfg4 leg: how the shared inputs reach the other GPUs (all: measure each, report the fastest)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output planes of the last timed step to DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3)
     wl = workload(args.workload)
     if args.impl == "reference":
@@ -577,6 +607,13 @@ def main():
     barrier()
     ms = e0.elapsed_time(e1)
     launches = r.stats()["kernel_launches"] - launches0
+    if args.dump_outputs:   # before the roofline and e2e legs below overwrite the output buffers
+        prefix = f"rank{rank}_" if world > 1 else ""
+        planes = {}
+        for k in range(n_out):
+            planes[f"{prefix}{out_ids[k].decode()}_y"] = out_y[k].cpu().numpy()
+            planes[f"{prefix}{out_ids[k].decode()}_uv"] = out_uv[k].cpu().numpy()
+        dump_outputs(args.dump_outputs, planes, DUMP_BYTES // world)
     ms_by_rank = [ms]
     if dist is not None:
         g = [torch.zeros(2, device=dev) for _ in range(world)]
